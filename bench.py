@@ -179,6 +179,13 @@ def gen_list(n_graphs, nbar=NBAR, seed=SEED, attr=0, as_adj=False):
     return out
 
 
+def dump_rows(n_rows, n_cols):
+    """Sorted, seeded sample of row indices for --dump-outputs: the same rows on every run with the same arguments,
+    few enough that their fp32 and fp64 copies stay under 48 MB together."""
+    k = int(min(n_rows, 256, max(1, 48e6 // (12 * n_cols))))
+    return np.sort(np.random.RandomState(20240).choice(n_rows, size=k, replace=False))
+
+
 def bind_to_gpu_node(torch, local):
     """Run this process on the CPUs of the NUMA node the GPU hangs off (what `numactl --cpunodebind` would do): host
     buffers the bench allocates (pinned CSR / K) then live next to the GPU's PCIe root.  Returns the node or None."""
@@ -297,16 +304,16 @@ def run_reference(args, rank, world):
     print(json.dumps(line), flush=True)
 
 
-def other_paths(eng, local, X2, with_cpu):
+def other_paths(eng, local, X2, with_cpu, steps):
     """BASELINE configs 3 (ShortestPath, 5 000 graphs, avg 60 nodes) and 5 (ShortestPathAttr, 2 000 graphs, d = 16) and
     WL-OA on the graphs of config 2: one GPU, CSR resident in HBM -> K resident in HBM, CUDA events on the engine's
-    stream; each with its dominant kernel against the stated roof (SURVEY 8d) and the real reference on a bounded
-    sample beside it."""
+    stream, `steps` timed steps each; each with its dominant kernel against the stated roof (SURVEY 8d) and the real
+    reference on a bounded sample beside it."""
     from grakel_b200.packing import label_ids, pack
     peak_tf, peak_hbm, _ = peaks()
     out = {}
 
-    def timed(fn, steps=10, warmup=3):
+    def timed(fn, warmup=3):
         for _ in range(warmup):
             st = fn()
         eng.event_record(4)
@@ -375,7 +382,7 @@ def other_paths(eng, local, X2, with_cpu):
         st = eng.spattr_features()
         eng.gram(n, out=False, dtype=np.float64, stats=st, want_diag=False)
         return st
-    ms, st = timed(step5, steps=5, warmup=2)
+    ms, st = timed(step5, warmup=2)
     D5 = int(st.n_columns)
     tf32_peak = peak_tf / 2.0
     fl = 2.0 * n * n * D5
@@ -498,7 +505,15 @@ def main():
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-paths", action="store_true", help="skip configs 3 / 5 / WL-OA")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed to DIR/<name>.npy: a seeded sample of rows of K from "
+                         "the device-resident pass (K_rows, fp32) and from the C-ABI end-to-end call (K_e2e_rows, fp64), "
+                         "their global row numbers (K_row_ids) and the whole diagonal (K_diag); rank 0's rows at N > 1")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of --impl b200")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
@@ -575,6 +590,15 @@ def main():
         dev_ms = eng.event_elapsed(0, 1)
         barrier()
         wall_ms = (time.perf_counter() - t0) * 1e3
+    dump, rows = None, None
+    if args.dump_outputs and rank == 0:
+        # K of the last timed step is still in the library-owned device buffer; later calls overwrite it
+        Kf = np.empty((re_ - rb, n), dtype=np.float32)
+        eng.fetch(Kf)
+        rows = dump_rows(re_ - rb, n)
+        dump = {"K_rows": Kf[rows], "K_row_ids": (rb + rows).astype(np.float64),
+                "K_diag": Kf[np.arange(re_ - rb), rb + np.arange(re_ - rb)]}
+        del Kf
     t_ms = torch.tensor([dev_ms], device="cuda")
     stages_per_rank = None
     if world > 1:
@@ -615,6 +639,8 @@ def main():
             per_step.append((time.perf_counter() - t1) * 1e3)
         barrier()
         e2e_t = torch.tensor([(time.perf_counter() - t0) / args.steps], device="cuda")
+        if dump is not None:
+            dump["K_e2e_rows"] = Kh[rows]  # before the breakdown below writes Kh again
         if world > 1:
             dist.all_reduce(e2e_t, op=dist.ReduceOp.MAX)
         e2e = {"value": n * n / float(e2e_t.item()), "unit": "pairs/s",
@@ -660,7 +686,7 @@ def main():
         dist_check = {"row_blocks_equal_single_gpu_prefix": bool(okt.item() == 1), "prefix": p1}
         n4 = int(os.environ.get("GRAKEL_B200_CONFIG4_GRAPHS", "50000" if world == 8 else "0"))
         if n4 > 0:
-            config4 = run_config4(eng, n4, rank, world, local, dist, torch, _lib, max(3, min(args.steps, 5)))
+            config4 = run_config4(eng, n4, rank, world, local, dist, torch, _lib, args.steps)
 
     # ------------------------------------------------ end to end through the Python API (SURVEY 8d T_e2e)
     e2e_api, paths = None, None
@@ -694,7 +720,7 @@ def main():
                    "list_build_ms_not_timed": t_gen * 1e3}
         if not args.no_paths:
             try:
-                paths = other_paths(eng, local, X, not args.no_cpu)
+                paths = other_paths(eng, local, X, not args.no_cpu, args.steps)
             except Exception as e:  # the headline line must survive a failure of the secondary measurements
                 paths = {"error": repr(e)}
         del X
@@ -781,6 +807,11 @@ def main():
     if not args.no_cpu and world == 1:
         os.sched_setaffinity(0, all_cpus)  # the CPU leg may use every core of the box
         line["cpu_baseline"] = cpu_baseline_obj(cpu_arm(steps=1, budget_s=12.0), n)
+    if dump is not None:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in dump.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), np.ascontiguousarray(a))
+        print("bench: wrote %s to %s" % (", ".join(sorted(dump)), args.dump_outputs), file=sys.stderr)
     print(json.dumps(line), file=real_stdout, flush=True)
     if world > 1:
         leave()

@@ -14,9 +14,6 @@ import numpy as np
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.join(HERE, "..", "..")
-sys.path.insert(0, os.environ.get("GRAKEL_REF", os.path.join(ROOT, "baseline", "_ref")))
-
-from grakel import ShortestPath, ShortestPathAttr, WeisfeilerLehman  # noqa: E402  (the reference)
 
 
 def gen_real(n_graphs, nbar, seed, attr=0):
@@ -42,6 +39,9 @@ def gen_real(n_graphs, nbar, seed, attr=0):
 
 
 if __name__ == "__main__":
+    # the reference is imported only to write the fixtures: the tests import gen_real from here without it
+    sys.path.insert(0, os.environ.get("GRAKEL_REF", os.path.join(ROOT, "baseline", "_ref")))
+    from grakel import ShortestPath, ShortestPathAttr, WeisfeilerLehman  # (the reference)
     warnings.simplefilter("ignore")
     out = {}
     X = gen_real(40, 12, 21)

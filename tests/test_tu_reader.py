@@ -2,11 +2,13 @@
 fast path of the estimators.
 
 CPU (-m "not gpu"): the native reader against (a) the oracle's restatement of read_data, (b) digests of the REAL
-reference's read_data on its own bundled datasets (tests/golden/tu_digest.json, checked when /root/reference is
-present), (c) the reference's MUTAG kernel matrices through the numpy model of the device pipeline.
+reference's read_data on its own bundled datasets (tests/golden/tu_digest.json; the MUTAG and Cuneiform files are
+stored in tests/golden/tu_datasets.tar.xz), (c) the reference's MUTAG kernel matrices through the numpy model of the
+device pipeline.
 GPU (-m gpu): estimators fed with blocks read from files against the same goldens."""
 import json
 import os
+import tarfile
 
 import numpy as np
 import pytest
@@ -22,7 +24,6 @@ from oracle.gk_oracle import WLOAOracle, gen, read_data_oracle, tu_digest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 G = os.path.join(ROOT, "tests", "golden")
-REF_DATA = "/root/reference/grakel/tests/data"
 
 
 def _mutag():
@@ -57,6 +58,16 @@ def mutag_dir(tmp_path_factory):
     return str(d)
 
 
+@pytest.fixture(scope="module")
+def bundled_dir(tmp_path_factory):
+    """The reference's bundled MUTAG and Cuneiform datasets (tests/data of ysig/GraKeL, without Cuneiform's edge
+    attributes, which read_data does not read), extracted from tests/golden/tu_datasets.tar.xz."""
+    d = tmp_path_factory.mktemp("bundled")
+    with tarfile.open(os.path.join(G, "tu_datasets.tar.xz")) as t:
+        t.extractall(d, filter="data")
+    return str(d)
+
+
 # ------------------------------------------------------------------ reader vs read_data
 @pytest.mark.parametrize("kernel,mode", [("WL", "wl"), ("SP", "sp")])
 def test_reader_matches_the_read_data_restatement(mutag_dir, kernel, mode):
@@ -67,24 +78,23 @@ def test_reader_matches_the_read_data_restatement(mutag_dir, kernel, mode):
     assert got.data.mode == mode and got.data.n_graphs == 188
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_DATA), reason="the reference's bundled datasets are only in the build container")
 @pytest.mark.parametrize("name", ["MUTAG", "Cuneiform"])
 @pytest.mark.parametrize("sym", [False, True])
 @pytest.mark.parametrize("attr", [False, True])
-def test_reader_matches_the_real_reference_on_its_bundled_datasets(name, sym, attr):
+def test_reader_matches_the_real_reference_on_its_bundled_datasets(bundled_dir, name, sym, attr):
     gold = json.load(open(os.path.join(G, "tu_digest.json")))[f"{name}_sym{int(sym)}_attr{int(attr)}"]
     if "error" in gold:  # Cuneiform's two-column node_labels.txt: int() raises ValueError in read_data
         with pytest.raises(ValueError):
-            read_tu(REF_DATA, name, kernel="WL", is_symmetric=sym, prefer_attr_nodes=attr)
+            read_tu(bundled_dir, name, kernel="WL", is_symmetric=sym, prefer_attr_nodes=attr)
         return
     for kernel, mode in (("WL", "wl"), ("SP", "sp")):
-        got = read_tu(REF_DATA, name, kernel=kernel, is_symmetric=sym, prefer_attr_nodes=attr)
+        got = read_tu(bundled_dir, name, kernel=kernel, is_symmetric=sym, prefer_attr_nodes=attr)
         assert got.data.n_graphs == gold["graphs"]
         assert tu_digest(_elements_of(got, mode), mode) == gold[mode]
         assert int(got.target.sum()) == gold["classes_sum"]
         assert len(got.edge_labels) == gold["edge_label_entries"] and int(got.edge_labels.sum()) == gold["edge_label_sum"]
     # and the oracle's restatement of read_data agrees with the real one
-    ref, _ = read_data_oracle(REF_DATA, name, is_symmetric=sym, prefer_attr_nodes=attr)
+    ref, _ = read_data_oracle(bundled_dir, name, is_symmetric=sym, prefer_attr_nodes=attr)
     assert tu_digest(ref, "wl") == gold["wl"] and tu_digest(ref, "sp") == gold["sp"]
 
 
