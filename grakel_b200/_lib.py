@@ -20,6 +20,7 @@ GK_NORMALIZE, GK_NAN_TO_NUM, GK_GRAM_SIMT, GK_OUT_DEVICE, GK_FULL_TILES, GK_DENS
 GK_DIST, GK_DIST_GATHER = 64, 128
 GK_SP_WITH_LABELS, GK_SP_KEEP_DIST, GK_SP_DIJKSTRA_ORDER = 1, 2, 4
 GK_ERR_RANGE, GK_ERR_UNSUPPORTED = -4, -5
+GK_NH_COUNT_SENSITIVE = 1
 
 
 class GkStats(C.Structure):
@@ -60,6 +61,9 @@ _SYMBOLS = {
     "gk_spattr_features": (C.c_int, [_P, C.c_int32, C.POINTER(GkStats)]),
     "gk_wl_sp_features": (C.c_int, [_P, C.c_int32, C.c_int32, C.POINTER(GkStats)]),
     "gk_wl_oa_features": (C.c_int, [_P, C.c_int32, C.POINTER(GkStats)]),
+    "gk_nh_features": (C.c_int, [_P, C.c_int32, C.c_int32, C.c_int32, _P, C.POINTER(GkStats)]),
+    "gk_nh_gram": (C.c_int, [_P, C.c_int64, C.c_int32, _P, C.c_int32, C.c_int64, C.POINTER(GkStats)]),
+    "gk_nh_labels": (C.c_int, [_P, C.c_int32, _P]),
     "gk_gram": (C.c_int, [_P, C.c_int64, C.c_int32, C.c_int64, C.c_int64, _P, C.c_int32, C.c_int64, _P, _P,
                           C.POINTER(GkStats)]),
     "gk_fetch": (C.c_int, [_P, _P, C.c_int32, C.c_int64]),
@@ -224,6 +228,44 @@ class Engine:
         with self._lock:
             self._check(self.lib.gk_wl_oa_features(self.h, int(n_iter), C.byref(st)))
         return st
+
+    def nh_features(self, R, bits, count_sensitive, labels0):
+        """NeighborhoodHash levels of the packed block; labels0 = int64 hashed level-0 label per vertex, -1 = None."""
+        st = GkStats()
+        lab = np.ascontiguousarray(labels0, dtype=np.int64)
+        with self._lock:
+            self._check(self.lib.gk_nh_features(self.h, int(R), int(bits), GK_NH_COUNT_SENSITIVE if count_sensitive else 0,
+                                                _ptr(lab), C.byref(st)))
+        return st
+
+    def nh_gram(self, n_graphs, n_fit=None, out=None, simt=False, dense_all=False, device_ptr=None, ld=0, stats=None):
+        """fp64 NeighborhoodHash matrix: a fresh host array, `out`, `device_ptr` (raw device pointer) or, with
+        out=False, left on the device (result_device / fetch)."""
+        n_fit = n_graphs if n_fit is None else int(n_fit)
+        rows = n_graphs if n_fit == n_graphs else n_graphs - n_fit
+        flags = (GK_GRAM_SIMT if simt else 0) | (GK_DENSE_ALL if dense_all else 0)
+        K, kptr = None, None
+        if device_ptr is not None:
+            flags |= GK_OUT_DEVICE
+            kptr = C.c_void_p(int(device_ptr))
+        elif out is None:
+            K = host_matrix(rows, n_fit, np.float64)
+            kptr = _ptr(K)
+        elif out is not False:
+            K = out
+            assert K.dtype == np.float64 and K.flags.c_contiguous and K.shape == (rows, n_fit)
+            kptr = _ptr(K)
+        st = stats if stats is not None else GkStats()
+        with self._lock:
+            self._check(self.lib.gk_nh_gram(self.h, n_fit, flags, kptr, GK_F64, int(ld), C.byref(st)))
+        return K
+
+    def nh_labels(self, level, n_vertices):
+        """u64 labels of one level (2^64 - 1 = None)."""
+        out = np.empty(n_vertices, dtype=np.uint64)
+        with self._lock:
+            self._check(self.lib.gk_nh_labels(self.h, int(level), _ptr(out)))
+        return out
 
     def sp_features(self, with_labels=True, keep_dist=False, dijkstra_order=False):
         st = GkStats()

@@ -25,7 +25,10 @@
 #include "wl_fused.cuh"
 #include "wl_fused2.cuh"
 #include "wl_oa.cuh"
+#include "nh.cuh"
 #include "tu_reader.h"
+#include <cub/device/device_radix_sort.cuh>
+#include <cub/device/device_scan.cuh>
 #include "comm.h"
 
 namespace gk {
@@ -132,6 +135,8 @@ struct HandleExtra {
   long long tiles_key[8] = {-1, -1, -1, -1, -1, -1, -1, -1};
   long long tiles_n = 0;
   long long head_dc_pad = 0;  // panel width of the last pass whose threshold came from the cost model (not GK_DENSE_ALL / FORCE_T)
+  // gk_nh_features: per level, the expanded block's columns and entries (what gk_nh_gram hands to gk_gram)
+  std::vector<long long> nh_cols, nh_entries;
 };
 static std::vector<std::pair<gk_handle*, HandleExtra*>> g_extra;
 static HandleExtra* extra_of(gk_handle* h) {
@@ -286,7 +291,8 @@ int gk_destroy(gk_handle* h) {
                         &h->tail_ent, &h->tail_cur, &h->part_max, &h->part_new, &h->diag_u64, &h->diag_f64, &h->panel,
                         &h->sp_dist, &h->sp_dict_keys, &h->sp_dict_ids, &h->sp_dkeys, &h->sp_graph_off, &h->fattr, &h->tiles,
                         &h->K, &h->K_stage, &h->wlf_buf, &h->row_map, &h->diag_rows, &h->oa_keys, &h->oa_cnt, &h->oa_colcnt, &h->wl_single,
-                        &h->diag_frozen, &h->sp_lists, &h->wl_payload, &h->gram_dyn, &h->tb_cnt, &h->tb_ent, &h->tb_ovf};
+                        &h->diag_frozen, &h->sp_lists, &h->wl_payload, &h->gram_dyn, &h->tb_cnt, &h->tb_ent, &h->tb_ovf,
+                        &h->nh_labels, &h->nh_keys, &h->nh_cnt, &h->nh_colcnt, &h->nh_diag, &h->nh_tmp, &h->nh_kf};
   for (auto* b : bufs) b->release();
   h->h_scalars.release();
   h->h_colstats.release();
@@ -980,6 +986,262 @@ int gk_wl_labels(gk_handle* h, int32_t level, int32_t* out) {
     src = h->slot_of.as<int>();
   }
   GK_CUDA(cudaMemcpyAsync(out, src, h->V * 4, cudaMemcpyDeviceToHost, h->stream));
+  GK_CUDA(cudaStreamSynchronize(h->stream));
+  return GK_OK;
+}
+
+// ---------------------------------------------------------------------------
+// NeighborhoodHash (nh.cuh).  gk_nh_features: the R relabel levels, then per level the histogram of the non-None
+// labels (dense column ids of the labels present) and its unary expansion (wl_oa.cuh), kept for gk_nh_gram.
+static size_t align256(size_t x) { return (x + 255) / 256 * 256; }
+
+int gk_nh_features(gk_handle* h, int32_t R, int32_t bits, int32_t flags, const int64_t* labels0, gk_stats* stats) {
+  if (!h) return fail(GK_ERR_ARG, "null handle");
+  if (h->N <= 0) return fail(GK_ERR_STATE, "gk_nh_features: no graphs packed");
+  if (R < 1 || R >= MAX_LEVELS) return fail(GK_ERR_ARG, "gk_nh_features: R out of range");
+  if (bits < 1 || bits > 63) return fail(GK_ERR_ARG, "gk_nh_features: bits must be in 1 .. 63");
+  const int64_t V = h->V, N = h->N;
+  if (V > 0 && !labels0) return fail(GK_ERR_ARG, "gk_nh_features: labels0 is required");
+  GK_CUDA(cudaSetDevice(h->dev));
+  const int64_t launches0 = h->launches;
+  h->features_ready = false; h->feat_serial++;
+  h->feature_kind = 0;
+  const size_t Vs = (size_t)std::max<int64_t>(V, 1);
+  const unsigned long long mask = (1ULL << bits) - 1ULL;
+  const bool cs = flags & GK_NH_COUNT_SENSITIVE;
+  GK_TRY(h->nh_labels.ensure((size_t)(R + 1) * Vs * 8));
+  GK_TRY(h->nh_keys.ensure((size_t)R * Vs * 8));
+  GK_TRY(h->nh_cnt.ensure((size_t)R * Vs * 4));
+  GK_TRY(h->nh_colcnt.ensure((size_t)R * (Vs + 1) * 4));
+  GK_TRY(h->nh_diag.ensure((size_t)R * N * 8));
+  unsigned long long* lab = h->nh_labels.as<unsigned long long>();
+  // scratch: sorted labels | sorted graph ids | flags | scan | count-block keys | counts | run starts | per-level
+  // counters + cursors | CUB temporary storage
+  size_t sort_tmp = 0, scan_tmp = 0;
+  GK_CUDA(cub::DeviceRadixSort::SortPairs(nullptr, sort_tmp, (const unsigned long long*)nullptr, (unsigned long long*)nullptr,
+                                          (const int*)nullptr, (int*)nullptr, (int)Vs, 0, 64, h->stream));
+  GK_CUDA(cub::DeviceScan::ExclusiveSum(nullptr, scan_tmp, (const unsigned long long*)nullptr, (unsigned long long*)nullptr,
+                                        (int)Vs, h->stream));
+  const size_t o_sg = align256(Vs * 8), o_flag = o_sg + align256(Vs * 4), o_pos = o_flag + align256(Vs * 8),
+               o_ck = o_pos + align256(Vs * 8), o_cc = o_ck + align256(Vs * 8), o_first = o_cc + align256(Vs * 4),
+               o_small = o_first + align256((Vs + 1) * 4),
+               o_cub = o_small + align256((size_t)R * (sizeof(NhLevelCounts) + sizeof(OaCursors))),
+               tmp_bytes = o_cub + std::max(sort_tmp, scan_tmp);
+  GK_TRY(h->nh_tmp.ensure(tmp_bytes));
+  char* tb = h->nh_tmp.as<char>();
+  unsigned long long* sk = reinterpret_cast<unsigned long long*>(tb);
+  int* sg = reinterpret_cast<int*>(tb + o_sg);
+  unsigned long long* flag = reinterpret_cast<unsigned long long*>(tb + o_flag);
+  unsigned long long* pos = reinterpret_cast<unsigned long long*>(tb + o_pos);
+  unsigned long long* ck = reinterpret_cast<unsigned long long*>(tb + o_ck);
+  unsigned* cc = reinterpret_cast<unsigned*>(tb + o_cc);
+  int* first = reinterpret_cast<int*>(tb + o_first);
+  NhLevelCounts* lc = reinterpret_cast<NhLevelCounts*>(tb + o_small);
+  OaCursors* oc = reinterpret_cast<OaCursors*>(tb + o_small + (size_t)R * sizeof(NhLevelCounts));
+  void* cub_tmp = tb + o_cub;
+  GK_TRY(h->colmin.ensure(Vs * 4));  // largest count / first threshold column of every count-block column
+  GK_TRY(h->colmax.ensure(Vs * 4));
+  DevScalars* sc = h->scalars.as<DevScalars>();
+
+  GK_CUDA(cudaEventRecord(h->tev[2], h->stream));
+  if (V) GK_CUDA(cudaMemcpyAsync(lab, labels0, V * 8, cudaMemcpyHostToDevice, h->stream));  // -1 = all ones = None
+  for (int r = 1; r <= R && V; ++r) {  // slot r = level r - 1 = NH_ applied r times (:196-198)
+    const unsigned long long* in = lab + (size_t)(r - 1) * V;
+    unsigned long long* out = lab + (size_t)r * V;
+    const int width = h->group_width;  // wider rows are in the packed large list
+    if (cs) nh_relabel<true><<<cdiv(V, 256), 256, 0, h->stream>>>((int)V, width, h->row_ptr.as<int>(), h->col_idx.as<int>(), in, out, bits, mask);
+    else nh_relabel<false><<<cdiv(V, 256), 256, 0, h->stream>>>((int)V, width, h->row_ptr.as<int>(), h->col_idx.as<int>(), in, out, bits, mask);
+    LAUNCH_CHECK(h);
+    if (h->n_large) {
+      const int grid = cdiv(h->n_large * 32, 256);
+      if (cs) nh_relabel_warp<true><<<grid, 256, 0, h->stream>>>((int)h->n_large, h->large_list.as<int>(), h->row_ptr.as<int>(), h->col_idx.as<int>(), in, out, bits, mask);
+      else nh_relabel_warp<false><<<grid, 256, 0, h->stream>>>((int)h->n_large, h->large_list.as<int>(), h->row_ptr.as<int>(), h->col_idx.as<int>(), in, out, bits, mask);
+      LAUNCH_CHECK(h);
+    }
+  }
+  GK_CUDA(cudaEventRecord(h->tev[3], h->stream));
+
+  GK_CUDA(cudaMemsetAsync(tb + o_small, 0, (size_t)R * (sizeof(NhLevelCounts) + sizeof(OaCursors)), h->stream));
+  GK_CUDA(cudaMemsetAsync(&sc->ft_overflow, 0, sizeof(unsigned), h->stream));
+  GK_CUDA(cudaMemsetAsync(h->nh_keys.p, 0xFF, (size_t)R * Vs * 8, h->stream));
+  GK_CUDA(cudaMemsetAsync(h->nh_colcnt.p, 0, (size_t)R * (Vs + 1) * 4, h->stream));
+  GK_CUDA(cudaMemsetAsync(h->nh_diag.p, 0, (size_t)R * N * 8, h->stream));
+  for (int r = 0; r < R && V; ++r) {
+    size_t t1 = sort_tmp;
+    GK_CUDA(cub::DeviceRadixSort::SortPairs(cub_tmp, t1, lab + (size_t)(r + 1) * V, sk, h->vgraph.as<int>(), sg, (int)V, 0, 64,
+                                            h->stream));
+    h->launches++;
+    nh_mark<<<cdiv(V, 256), 256, 0, h->stream>>>((int)V, sk, sg, flag);
+    LAUNCH_CHECK(h);
+    size_t t2 = scan_tmp;
+    GK_CUDA(cub::DeviceScan::ExclusiveSum(cub_tmp, t2, flag, pos, (int)V, h->stream));
+    h->launches++;
+    GK_CUDA(cudaMemsetAsync(ck, 0xFF, (size_t)V * 8, h->stream));
+    nh_emit<<<cdiv(V, 256), 256, 0, h->stream>>>((int)V, sk, sg, flag, pos, ck, first, lc + r);
+    LAUNCH_CHECK(h);
+    nh_counts<<<cdiv(V, 256), 256, 0, h->stream>>>((int)V, first, lc + r, cc);
+    LAUNCH_CHECK(h);
+    // unary expansion of the count block: one entry per non-None vertex (gk_wl_oa_features does the same for WL)
+    unsigned* colmaxcnt = h->colmin.as<unsigned>();
+    unsigned* colbase = h->colmax.as<unsigned>();
+    GK_CUDA(cudaMemsetAsync(colmaxcnt, 0, (size_t)V * 4, h->stream));
+    oa_colmax<<<h->sm_count * 8, 256, 0, h->stream>>>((size_t)V, ck, cc, colmaxcnt);
+    LAUNCH_CHECK(h);
+    oa_colbase<<<cdiv(V, OA_THREADS), OA_THREADS, 0, h->stream>>>(V, colmaxcnt, colbase, oc + r);
+    LAUNCH_CHECK(h);
+    oa_expand<<<cdiv(V, OA_THREADS), OA_THREADS, 0, h->stream>>>(
+        (size_t)V, ck, cc, colbase, (size_t)V, h->nh_keys.as<unsigned long long>() + (size_t)r * Vs,
+        h->nh_cnt.as<unsigned>() + (size_t)r * Vs, oc + r, h->nh_colcnt.as<unsigned>() + (size_t)r * (Vs + 1),
+        h->nh_diag.as<unsigned long long>() + (size_t)r * N, sc);
+    LAUNCH_CHECK(h);
+  }
+  GK_CUDA(cudaEventRecord(h->ev[13], h->stream));
+  std::vector<NhLevelCounts> hl(R);
+  std::vector<OaCursors> ho(R);
+  GK_CUDA(cudaMemcpyAsync(hl.data(), lc, (size_t)R * sizeof(NhLevelCounts), cudaMemcpyDeviceToHost, h->stream));
+  GK_CUDA(cudaMemcpyAsync(ho.data(), oc, (size_t)R * sizeof(OaCursors), cudaMemcpyDeviceToHost, h->stream));
+  DevScalars* hs;
+  GK_TRY(read_scalars(h, &hs));
+  if (hs->ft_overflow) return fail(GK_ERR_STATE, "gk_nh_features: expanded feature block overflow");
+  HandleExtra* ex = extra_of(h);
+  ex->nh_cols.assign(R, 0);
+  ex->nh_entries.assign(R, 0);
+  int64_t tot_cols = 0, tot_ent = 0;
+  for (int r = 0; r < R; ++r) {
+    ex->nh_cols[r] = (long long)ho[r].n_cols;
+    ex->nh_entries[r] = (long long)ho[r].n_entries;
+    tot_cols += ex->nh_cols[r];
+    tot_ent += ex->nh_entries[r];
+  }
+  h->nh_R = R;
+  h->n_levels = R;
+  h->feature_kind = 4;
+  if (stats) {
+    memset(stats, 0, sizeof(*stats));
+    stats->n_graphs = N; stats->n_vertices = V; stats->n_edges = h->E;
+    stats->n_levels = R;
+    for (int r = 0; r < R; ++r) stats->level_dims[r] = (int64_t)hl[r].n_cols;
+    stats->n_columns = tot_cols;
+    stats->n_entries = tot_ent;
+    stats->kernel_launches = h->launches - launches0;
+    stats->ms_features = ev_ms(h->tev[2], h->tev[3]);
+    stats->ms_panel = ev_ms(h->tev[3], h->ev[13]);
+  }
+  return GK_OK;
+}
+
+// gk_gram over level r's expanded block: the handle's feature-block buffers are pointed at the level's slices for the
+// call and restored afterwards (gk_gram reads them, it never reallocates them)
+static int nh_level_gram(gk_handle* h, int r, int64_t n_fit, int32_t flags, float* d_kf, int64_t ldf, gk_stats* gs) {
+  const size_t Vs = (size_t)std::max<int64_t>(h->V, 1);
+  HandleExtra* ex = extra_of(h);
+  DevBuf lk, lc, lcc, ld;
+  lk.p = h->nh_keys.as<unsigned long long>() + (size_t)r * Vs; lk.cap = Vs * 8;
+  lc.p = h->nh_cnt.as<unsigned>() + (size_t)r * Vs; lc.cap = Vs * 4;
+  lcc.p = h->nh_colcnt.as<unsigned>() + (size_t)r * (Vs + 1); lcc.cap = (Vs + 1) * 4;
+  ld.p = h->nh_diag.as<unsigned long long>() + (size_t)r * h->N; ld.cap = (size_t)h->N * 8;
+  GK_TRY(h->part_max.ensure(4));
+  GK_TRY(h->part_new.ensure(4));
+  nh_parts<<<1, 1, 0, h->stream>>>((unsigned long long)ex->nh_entries[r], h->part_max.as<unsigned>(), h->part_new.as<unsigned>());
+  LAUNCH_CHECK(h);
+  const size_t ft_cap0 = h->ft_cap;
+  const int64_t col_cap0 = h->col_cap, n_columns0 = h->n_columns, n_part0 = h->n_part;
+  std::swap(h->ft_keys, lk); std::swap(h->ft_cnt, lc); std::swap(h->colcnt, lcc); std::swap(h->diag_u64, ld);
+  h->ft_cap = Vs; h->col_cap = (int64_t)Vs + 1; h->n_columns = ex->nh_cols[r]; h->n_part = 1;
+  h->features_ready = true; h->feat_serial++;
+  const int rc = gk_gram(h, n_fit, GK_OUT_DEVICE | (flags & (GK_GRAM_SIMT | GK_DENSE_ALL)), 0, -1, d_kf, GK_F32, ldf,
+                         nullptr, nullptr, gs);
+  std::swap(h->ft_keys, lk); std::swap(h->ft_cnt, lc); std::swap(h->colcnt, lcc); std::swap(h->diag_u64, ld);
+  h->ft_cap = ft_cap0; h->col_cap = col_cap0; h->n_columns = n_columns0; h->n_part = n_part0;
+  h->features_ready = false; h->feat_serial++;
+  return rc;
+}
+
+int gk_nh_gram(gk_handle* h, int64_t n_fit, int32_t flags, void* K_out, int32_t out_dtype, int64_t ld, gk_stats* stats) {
+  if (!h) return fail(GK_ERR_ARG, "null handle");
+  if (h->feature_kind != 4 || h->nh_R < 1) return fail(GK_ERR_STATE, "gk_nh_gram: no NeighborhoodHash levels (call gk_nh_features)");
+  if (out_dtype != GK_F64) return fail(GK_ERR_UNSUPPORTED, "gk_nh_gram: the NeighborhoodHash Gram is fp64 only");
+  if (h->n_rows > 0) return fail(GK_ERR_UNSUPPORTED, "gk_nh_gram: row map with NeighborhoodHash levels");
+  if (flags & (GK_NORMALIZE | GK_DIST | GK_DIST_GATHER)) return fail(GK_ERR_UNSUPPORTED, "gk_nh_gram: unsupported flag");
+  const int64_t N = h->N;
+  if (n_fit <= 0 || n_fit > N) return fail(GK_ERR_ARG, "gk_nh_gram: n_fit out of range");
+  // level intersections are fp32 integers: exact while every graph has fewer than 2^24 vertices
+  if (h->max_graph_size >= (1 << 24)) return fail(GK_ERR_RANGE, "gk_nh_gram: a graph with 2^24 or more vertices");
+  GK_CUDA(cudaSetDevice(h->dev));
+  const bool square = n_fit == N;
+  const int64_t rows = square ? N : N - n_fit, cols = n_fit;
+  const int row0 = square ? 0 : (int)n_fit;
+  const bool dev_out = flags & GK_OUT_DEVICE;
+  if (dev_out && !K_out) return fail(GK_ERR_ARG, "gk_nh_gram: GK_OUT_DEVICE without a pointer");
+  if (ld <= 0) ld = cols;
+  if (ld < cols) return fail(GK_ERR_ARG, "gk_nh_gram: ld smaller than the row length");
+  const int64_t launches0 = h->launches;
+  const int64_t ldf = (cols + 7) / 8 * 8;  // 32-byte rows: TMA stores of the level Gram
+  const int R = h->nh_R;
+  const size_t level_stride = (size_t)std::max<int64_t>(rows, 1) * ldf;  // the R level Grams side by side
+  GK_TRY(h->nh_kf.ensure((size_t)R * level_stride * 4));
+  double* K64;
+  int64_t ldk;
+  if (dev_out) {
+    K64 = reinterpret_cast<double*>(K_out);
+    ldk = ld;
+  } else {  // library-owned result (gk_result_device / gk_fetch)
+    GK_TRY(h->K.ensure((size_t)std::max<int64_t>(rows, 1) * cols * 8));
+    K64 = h->K.as<double>();
+    ldk = cols;
+    h->K_rows = rows; h->K_cols = cols; h->K_ld = cols; h->K_dtype = GK_F64;
+  }
+  gk_stats gs;
+  memset(&gs, 0, sizeof(gs));
+  float ms_gram = 0.f, ms_comb = 0.f;
+  for (int r = 0; r < R && rows > 0; ++r) {
+    memset(&gs, 0, sizeof(gs));
+    GK_TRY(nh_level_gram(h, r, n_fit, flags, h->nh_kf.as<float>() + (size_t)r * level_stride, ldf, &gs));
+    ms_gram += gs.ms_total;
+  }
+  if (rows > 0) {
+    GK_CUDA(cudaEventRecord(h->tev[0], h->stream));
+    nh_combine<<<h->sm_count * 8, 256, 0, h->stream>>>(rows, cols, row0, h->graph_ptr.as<int>(), h->nh_kf.as<float>(), ldf,
+                                                       (long long)level_stride, R, K64, ldk);
+    LAUNCH_CHECK(h);
+    GK_CUDA(cudaEventRecord(h->tev[1], h->stream));
+    GK_CUDA(cudaEventSynchronize(h->tev[1]));
+    ms_comb = ev_ms(h->tev[0], h->tev[1]);
+  }
+  h->feature_kind = 4;  // the levels stay usable (a second gk_nh_gram, gk_nh_labels)
+  GK_CUDA(cudaEventRecord(h->ev[14], h->stream));
+  if (K_out && !dev_out && rows > 0)
+    GK_CUDA(cudaMemcpy2DAsync(K_out, (size_t)ld * 8, K64, (size_t)ldk * 8, (size_t)cols * 8, (size_t)rows,
+                              cudaMemcpyDeviceToHost, h->stream));
+  GK_CUDA(cudaEventRecord(h->ev[15], h->stream));
+  GK_CUDA(cudaStreamSynchronize(h->stream));
+  if (stats) {
+    const gk_stats last = gs;
+    memset(stats, 0, sizeof(*stats));
+    stats->n_graphs = N; stats->n_vertices = h->V; stats->n_edges = h->E;
+    stats->n_levels = R;
+    stats->n_dense_columns = last.n_dense_columns;
+    stats->n_tail_columns = last.n_tail_columns;
+    stats->threshold = last.threshold;
+    stats->gram_path = last.gram_path;
+    stats->max_diag = last.max_diag;
+    stats->gemm_tiles = last.gemm_tiles;
+    stats->kernel_launches = h->launches - launches0;
+    stats->ms_gemm = ms_gram;
+    stats->ms_tail = ms_comb;
+    stats->ms_d2h = ev_ms(h->ev[14], h->ev[15]);
+    stats->ms_total = ms_gram + ms_comb + stats->ms_d2h;
+  }
+  return GK_OK;
+}
+
+int gk_nh_labels(gk_handle* h, int32_t level, uint64_t* out) {
+  if (!h || !out) return fail(GK_ERR_ARG, "gk_nh_labels: null argument");
+  if (h->feature_kind != 4 || level < 0 || level >= h->nh_R) return fail(GK_ERR_STATE, "gk_nh_labels: no such level");
+  GK_CUDA(cudaSetDevice(h->dev));
+  if (h->V)
+    GK_CUDA(cudaMemcpyAsync(out, h->nh_labels.as<unsigned long long>() + (size_t)(level + 1) * h->V, h->V * 8,
+                            cudaMemcpyDeviceToHost, h->stream));
   GK_CUDA(cudaStreamSynchronize(h->stream));
   return GK_OK;
 }

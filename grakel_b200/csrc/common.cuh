@@ -159,9 +159,14 @@ struct gk_handle {
   int64_t pro_serial = -1;   // feat_serial for which gk_wl_features already ran the Gram prologue (square case):
                              // self similarities finished, column histogram on the host -- gk_gram then needs no
                              // host synchronisation before its launches
-  int feature_kind = 0;  // 1 = WL, 2 = SP, 3 = SP-attr (dense fp32 features)
+  int feature_kind = 0;  // 1 = WL, 2 = SP, 3 = SP-attr (dense fp32 features), 4 = NeighborhoodHash levels
 
   gk::DevBuf oa_keys, oa_cnt, oa_colcnt;  // WL-OA: unary-expanded block, swapped with ft_keys / ft_cnt / colcnt
+  // NeighborhoodHash (nh.cuh): u64 labels [R + 1][V] (slot 0 = hashed level-0 input), the R unary-expanded level
+  // blocks [R][V] keys / counts, [R][V + 1] graphs per column, [R][N] self similarities; sort / scan scratch; the fp32
+  // level Gram
+  gk::DevBuf nh_labels, nh_keys, nh_cnt, nh_colcnt, nh_diag, nh_tmp, nh_kf;
+  int nh_R = 0;
   // ---- columns / panel / diag
   gk::DevBuf colcnt, colmin, colmax, colslot, col_flags3, col_block_sums, colstats;
   int64_t col_cap = 0;  // allocated length of the per-column arrays

@@ -22,7 +22,8 @@ from . import _lib
 from .packing import Block
 
 _MODES = {"WL": 0, "VH": 0, "weisfeiler_lehman": 0, "vertex_histogram": 0, "subtree_wl": 0, "ST-WL": 0,
-          "SP": 1, "shortest_path": 1, "WL-OA": 1, "weisfeiler_lehman_optimal_assignment": 1}
+          "SP": 1, "shortest_path": 1, "WL-OA": 1, "weisfeiler_lehman_optimal_assignment": 1,
+          "NH": 1, "neighborhood_hash": 1}
 GK_TU_SYMMETRIC, GK_TU_ATTR_NODES, GK_TU_DEGREE_LABELS = 1, 2, 4
 
 
@@ -45,7 +46,7 @@ def read_tu(path, name, kernel="WL", with_classes=True, is_symmetric=False, pref
     `prefer_attr_nodes` loads node attributes instead of node labels (for ShortestPathAttr),
     `produce_labels_nodes` labels nodes by their degree when the dataset has no node labels."""
     if kernel not in _MODES:
-        raise ValueError("read_tu packs for WL / VH / SP / WL-OA; got " + repr(kernel))
+        raise ValueError("read_tu packs for WL / VH / SP / WL-OA / NH; got " + repr(kernel))
     mode = _MODES[kernel]
     lib = _lib.load_library()
 

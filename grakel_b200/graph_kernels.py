@@ -7,6 +7,8 @@ the kernels of the device hot path:
     "edge_histogram" / "EH"
     "core_framework" / "CORE"   (framework; base "shortest_path" or "weisfeiler_lehman" ...)
     "weisfeiler_lehman_optimal_assignment" / "WL-OA"
+    "neighborhood_hash" / "NH"  (R, nh_type, bits, random_state: the reference's dispatcher does not pass its own
+                                 random_state to this kernel, graph_kernels.py:524-525, so a seed goes in the dict)
 
 Any other reference kernel name raises NotImplementedError (not ValueError, which the reference reserves for
 unknown names).  The public surface (constructor parameters, `fit` / `transform` / `fit_transform`, the fitted
@@ -27,15 +29,15 @@ from sklearn.utils import check_random_state
 from sklearn.utils.validation import check_is_fitted
 
 from .core_framework import CoreFramework
-from .kernels import (EdgeHistogram, ShortestPath, ShortestPathAttr, VertexHistogram, WeisfeilerLehman,
-                      WeisfeilerLehmanOptimalAssignment)
+from .kernels import (EdgeHistogram, NeighborhoodHash, ShortestPath, ShortestPathAttr, VertexHistogram,
+                      WeisfeilerLehman, WeisfeilerLehmanOptimalAssignment)
 
 default_n_components = 100
 
 # reference names outside the hot path (graph_kernels.py:38-64)
 _OUTSIDE = frozenset((
     "random_walk", "RW", "graphlet_sampling", "GR", "subgraph_matching", "SM", "multiscale_laplacian", "ML",
-    "lovasz_theta", "LOVT", "svm_theta", "SVMT", "neighborhood_hash", "NH", "neighborhood_subgraph_pairwise_distance",
+    "lovasz_theta", "LOVT", "svm_theta", "SVMT", "neighborhood_subgraph_pairwise_distance",
     "NSPD", "odd_sth", "ODD", "propagation", "PR", "pyramid_match", "PM", "graph_hopper", "GH", "hadamard_code", "HC"))
 
 
@@ -50,6 +52,7 @@ for _names, _framework, _build in (
         (("edge_histogram", "EH"), False, lambda p: (EdgeHistogram, p)),
         (("weisfeiler_lehman_optimal_assignment", "WL-OA"), False, lambda p: (WeisfeilerLehmanOptimalAssignment, p)),
         (("shortest_path", "SP"), False, _shortest_path),
+        (("neighborhood_hash", "NH"), False, lambda p: (NeighborhoodHash, p)),
         (("weisfeiler_lehman", "WL"), True, lambda p: (WeisfeilerLehman, p)),
         (("core_framework", "CORE"), True, lambda p: (CoreFramework, p))):
     for _n in _names:
@@ -175,7 +178,8 @@ class GraphKernel(BaseEstimator, TransformerMixin):
         if entry is None:
             if name in _OUTSIDE:
                 raise NotImplementedError("kernel '" + str(name) + "' is outside the device hot path of grakel_b200 "
-                                          "(WL-subtree, vertex histogram, shortest path)")
+                                          "(WL-subtree, vertex histogram, edge histogram, shortest path, WL-OA, "
+                                          "neighborhood hash)")
             raise ValueError("Unsupported kernel: " + str(name))
         framework, build = entry
         if framework:

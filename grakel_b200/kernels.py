@@ -19,6 +19,7 @@ from collections.abc import Iterable
 import numpy as np
 from sklearn.base import BaseEstimator, TransformerMixin
 from sklearn.exceptions import NotFittedError
+from sklearn.utils import check_random_state
 from sklearn.utils.validation import check_is_fitted
 
 from . import _lib
@@ -872,3 +873,183 @@ class ShortestPathAttr(Kernel):
 
     def _device_features(self, eng):
         return eng.spattr_features(dijkstra_order=bool(getattr(self, "_dijkstra_order", False)))
+
+
+# ------------------------------------------------------------------------------
+_NH_ELEMENT_MSG = ("each element of X must be either a graph object or a list with at least a graph like object and "
+                   "node labels dict \n")
+
+
+def _nh_elements(X):
+    """The reference's element loop (neighborhood_hash.py:127-159, 272-313) without the graph work: yields the node-label
+    dict of every element that becomes a graph, warns on empty elements, raises as the reference does.
+
+    A one-member element warns and then reaches the graph tuple with the previous element's variables: the reference
+    fails there with UnboundLocalError for the first graph and AttributeError (a list has no `neighbors`) afterwards."""
+    i = 0
+    for idx, x in enumerate(X):
+        if isinstance(x, Graph):
+            x = x.as_element()
+        is_iter = isinstance(x, Iterable)
+        if is_iter:
+            x = list(x)
+        if not (is_iter and len(x) in (0, 1, 2, 3)):
+            raise TypeError(_NH_ELEMENT_MSG)
+        if len(x) == 0:
+            warnings.warn("Ignoring empty element on index: " + str(idx))
+            continue
+        if len(x) == 1:
+            warnings.warn("Ignoring empty element on index: " + str(i) + "\nLabels must be provided.")
+            if i == 0:
+                raise UnboundLocalError("cannot access local variable 'vertices' where it is not associated with a value")
+            raise AttributeError("'list' object has no attribute 'neighbors'")
+        i += 1
+        yield x[1]
+
+
+class NeighborhoodHash(Kernel):
+    """Neighborhood hashing kernel (neighborhood_hash.py:14-570, Hido & Kashima): every vertex label is hashed R times
+    from its own label and its out-neighbours' labels (a bit rotation and XORs, :367-504), and
+    K[i, j] = mean over the R levels of c_r / (n_i + n_j - c_r), c_r the multiset intersection of the two graphs' level-r
+    labels, n the vertex counts (:531-570).
+
+    The host builds the reference's label set and hash dictionary (:157, 164-189) with the same sequence of set
+    operations and RandomState draws, so `_labels_hash_dict` and `random_state_` end up as the reference leaves them;
+    the relabel levels, the per-level intersections (a unary-expanded histogram through the integer Gram) and the fp64
+    combine run on the device (`gk_nh_features` / `gk_nh_gram`).  `normalize` and `n_jobs` are accepted and have no
+    effect, as in the reference: the matrix is already normalised and `diagonal()` returns 1.0 (:343-365)."""
+
+    _graph_format = "dictionary"
+
+    def __init__(self, n_jobs=None, normalize=False, verbose=False, random_state=None, R=3, nh_type="simple", bits=8):
+        super().__init__(n_jobs=n_jobs, normalize=normalize, verbose=False)  # :50-52: verbose is dropped
+        self.random_state = random_state
+        self.R = R
+        self.nh_type = nh_type
+        self.bits = bits
+        self._initialized.update({"random_state": False, "R": False, "nh_type": False, "bits": False})
+
+    def initialize(self):
+        """:61-89"""
+        super().initialize()
+        if not self._initialized["random_state"]:
+            self.random_state_ = check_random_state(self.random_state)
+            self._initialized["random_state"] = True
+        if not self._initialized["R"]:
+            if type(self.R) is not int or self.R <= 0:
+                raise TypeError("R must be an intger bigger than zero")
+            self._initialized["R"] = True
+        if not self._initialized["nh_type"]:
+            if self.nh_type not in ("simple", "count_sensitive"):
+                raise TypeError("unrecognised neighborhood hashing type")
+            self._nh_cs = self.nh_type == "count_sensitive"
+            self._initialized["nh_type"] = True
+        if not self._initialized["bits"]:
+            if type(self.bits) is not int or self.bits <= 0:
+                raise TypeError("illegal number of bits for hashing")
+            self._max_number = 1 << self.bits
+            self._mask = self._max_number - 1
+            self._initialized["bits"] = True
+
+    # ---- host logic
+    def _pack(self, X):
+        """(block, per-graph label-value iterables in graph order) of a fit or transform input."""
+        if isinstance(X, Block):  # packed input (datasets.read_tu): the label set comes from the packed labels
+            block = X.require("sp", "wloa")
+            gp = block.graph_ptr
+            lab = block.labels.tolist() if isinstance(block.labels, np.ndarray) else list(block.labels)
+            return block, (lab[gp[g]:gp[g + 1]] for g in range(block.n_graphs))
+        if not isinstance(X, Iterable):
+            raise TypeError("input must be an iterable\n")
+        if type(X) is not list:
+            X = list(X)
+        label_dicts = list(_nh_elements(X))  # element checks, warnings and errors in the reference's order
+        if not label_dicts:
+            return None, ()
+        with warnings.catch_warnings():
+            warnings.simplefilter("ignore")  # the empty-element warnings were given above
+            block = pack(X, "wloa", len_ok=lambda n: n in (2, 3), type_error_msg=_NH_ELEMENT_MSG)
+        return block, (L.values() for L in label_dicts)
+
+    def _hash_labels(self, label_values):
+        """:157, 164-189: the label set, built with `|=` in graph order, zipped with draws from random_state_."""
+        labels_hash_set = set()
+        for vals in label_values:
+            labels_hash_set |= set(vals)
+        rs, M = self.random_state_, self._max_number
+        if len(labels_hash_set) > M:
+            warnings.warn("Number of labels is smaller than" "the biggest possible.. " "Collisions will appear on the "
+                          "new labels.")
+            nl, nrl = list(), len(labels_hash_set)
+            while nrl > M:
+                nl += rs.choice(M, M, replace=False).tolist()
+                nrl -= M
+            if nrl > 0:
+                nl += rs.choice(M, nrl, replace=False).tolist()
+        else:
+            nl = rs.choice(M, len(labels_hash_set), replace=False).tolist()
+        return dict(zip(labels_hash_set, nl))
+
+    @staticmethod
+    def _labels0(block, hash_dict):
+        """Hashed level-0 label of every packed vertex, -1 for a label outside the dictionary (None, :299)."""
+        labels = block.labels
+        if isinstance(labels, np.ndarray):
+            uniq, inv = np.unique(labels, return_inverse=True)
+            hv = np.fromiter((hash_dict.get(u, -1) for u in uniq.tolist()), dtype=np.int64, count=len(uniq))
+            return hv[inv.ravel()]
+        return np.fromiter((hash_dict.get(l, -1) for l in labels), dtype=np.int64, count=len(labels))
+
+    # ---- reference protocol
+    def fit(self, X, y=None):
+        """:91-206"""
+        self._method_calling = 1
+        self._is_transformed = False
+        self.initialize()
+        if X is None:
+            raise ValueError("`fit` input cannot be None")
+        block, label_values = self._pack(X)
+        if block is None:
+            raise ValueError("parsed input is empty")
+        self._labels_hash_dict = self._hash_labels(label_values)
+        self.X = Fitted(block, self._labels0(block, self._labels_hash_dict), self._labels_hash_dict)
+        return self
+
+    def fit_transform(self, X, y=None):
+        """:208-237"""
+        self._method_calling = 2
+        self.fit(X)
+        if np.any(np.diff(self.X.block.graph_ptr) == 0):
+            raise ZeroDivisionError("float division by zero")  # a graph without vertices against itself: 0 / 0.0
+        return self._run(self.X.block, self.X.ids, n_fit=self.X.block.n_graphs)
+
+    def transform(self, X):
+        """:239-322"""
+        self._method_calling = 3
+        check_is_fitted(self, ["X"])
+        if X is None:
+            raise ValueError("`transform` input cannot be None")
+        block, _ = self._pack(X)
+        self._is_transformed = True
+        n_fit = self.X.block.n_graphs
+        if block is None:  # the reference builds an empty matrix when every element was empty
+            return np.zeros((0, n_fit))
+        if np.any(np.diff(block.graph_ptr) == 0) and np.any(np.diff(self.X.block.graph_ptr) == 0):
+            raise ZeroDivisionError("float division by zero")
+        ids = np.concatenate([self.X.ids, self._labels0(block, self._labels_hash_dict)])
+        return self._run(Block.concat(self.X.block, block), ids, n_fit=n_fit)
+
+    def diagonal(self):
+        """:343-365: the matrix is normalised by construction."""
+        if getattr(self, "_is_transformed", False):
+            return 1.0, 1.0
+        return 1.0
+
+    def _run(self, block, labels0, n_fit):
+        """pack -> R relabel levels -> per-level intersections and the fp64 combine, all on the device."""
+        with _lib.engine(getattr(self, "device_", None)) as eng:
+            eng.pack(block.graph_ptr, block.row_ptr, block.col_idx)
+            self.stats_ = eng.nh_features(self.R, self.bits, self._nh_cs, labels0)
+            self.stats_gram_ = _lib.GkStats()
+            K = eng.nh_gram(block.n_graphs, n_fit=n_fit, stats=self.stats_gram_)
+        return K

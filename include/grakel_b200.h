@@ -27,6 +27,9 @@
  *   gk_wl_oa_features    WeisfeilerLehmanOptimalAssignment.parse_input + the O(N^2) Python loop of
  *                        histogram intersections (weisfeiler_lehman_optimal_assignment.py:78-229,
  *                        257-266, 433-437).
+ *   gk_nh_features, gk_nh_gram, gk_nh_labels
+ *                        NeighborhoodHash.fit / transform / pairwise_operation
+ *                        (neighborhood_hash.py:91-341, 392-570), see below.
  *   gk_spattr_features   ShortestPathAttr.parse_input + the bilinear pair kernel
  *                        (shortest_path.py:77-164) as an explicit feature map.
  *   gk_gram              VertexHistogram._calculate_kernel_matrix
@@ -142,6 +145,32 @@ int gk_wl_sp_features(gk_handle* h, int32_t n_iter, int32_t flags, gk_stats* sta
  * -- so that gk_gram's dot products are the histogram intersections sum_c min(Hs[i,c], Hs[j,c]) of
  * :257-266 / :433-437, the self similarities the row sums of :459-461, exactly (integers). */
 int gk_wl_oa_features(gk_handle* h, int32_t n_iter, gk_stats* stats);
+
+/* NeighborhoodHash (neighborhood_hash.py:91-206, 239-322, 324-341, 392-570).
+ *
+ * gk_nh_features replaces the R applications of NH_ (neighborhood_hash.py:191-201, 307-310: the simple hash of
+ * :392-418 or, with GK_NH_COUNT_SENSITIVE, the count-sensitive hash of :420-504) and prepares every level for the
+ * merge of nh_compare_labels (:531-570) as a unary-expanded histogram (the intersection c_r is a dot product).
+ *   labels0[V]  level-0 hashed label of every packed vertex (_labels_hash_dict[label], :189-194), -1 = None
+ *               (a transform label unseen at fit time, :299-300)
+ *   bits        1 .. 63 (the reference's `bits`, :83-88)
+ * stats: n_levels = R, level_dims[r] = distinct non-None labels of level r, n_columns / n_entries = columns / entries
+ * of the R expanded blocks, ms_features = the relabel, ms_panel = the level histograms and expansions.
+ *
+ * gk_nh_gram replaces pairwise_operation over all pairs (:324-341, kernel.py:257-284):
+ * K[i, j] = sum(a_0 .. a_{R-1}) / R with a_r = c_r / (double)(n_i + n_j - c_r), n = the graph's packed vertex count
+ * (None vertices included), the sum compensated as CPython's built-in sum() adds floats (Neumaier, CPython >= 3.12).  fp64 only.  n_fit == n_graphs: the square, symmetric fit_transform matrix;
+ * n_fit < n_graphs: [(n_graphs - n_fit) x n_fit], rows = Y graphs.  flags: GK_OUT_DEVICE (K_out is a device pointer,
+ * row pitch ld), GK_GRAM_SIMT / GK_DENSE_ALL select the path of the per-level integer Grams.  K_out == NULL keeps
+ * K on the device (gk_result_device / gk_fetch).  stats: ms_gemm = the R level Grams, ms_tail = the fp64 combine,
+ * ms_d2h = the copy to the host; gram_path / threshold / n_dense_columns are those of the last level.
+ *
+ * gk_nh_labels: the u64 labels of level `level` (0 .. R-1) per packed vertex, UINT64_MAX = None (tests). */
+#define GK_NH_COUNT_SENSITIVE 1
+int gk_nh_features(gk_handle* h, int32_t R, int32_t bits, int32_t flags, const int64_t* labels0, gk_stats* stats);
+int gk_nh_gram(gk_handle* h, int64_t n_fit, int32_t flags, void* K_out, int32_t out_dtype, int64_t ld,
+               gk_stats* stats);
+int gk_nh_labels(gk_handle* h, int32_t level, uint64_t* out);
 
 /* Gram matrix of the current feature block.
  *   n_fit == n_graphs : K is [n_graphs x n_graphs]                      (fit_transform)
