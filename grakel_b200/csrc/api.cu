@@ -289,7 +289,7 @@ int gk_destroy(gk_handle* h) {
                         &h->flags, &h->block_sums, &h->scalars, &h->ft_keys, &h->ft_cnt, &h->colcnt,
                         &h->colmin, &h->colmax, &h->colslot, &h->col_flags3, &h->col_block_sums, &h->colstats, &h->tail_desc,
                         &h->tail_ent, &h->tail_cur, &h->part_max, &h->part_new, &h->diag_u64, &h->diag_f64, &h->panel,
-                        &h->sp_dist, &h->sp_dict_keys, &h->sp_dict_ids, &h->sp_dkeys, &h->sp_graph_off, &h->fattr, &h->tiles,
+                        &h->sp_dist, &h->sp_dict_keys, &h->sp_dict_ids, &h->sp_dkeys, &h->sp_graph_off, &h->fattr, &h->fattr_exp, &h->tiles,
                         &h->K, &h->K_stage, &h->wlf_buf, &h->row_map, &h->diag_rows, &h->oa_keys, &h->oa_cnt, &h->oa_colcnt, &h->wl_single,
                         &h->diag_frozen, &h->sp_lists, &h->wl_payload, &h->gram_dyn, &h->tb_cnt, &h->tb_ent, &h->tb_ovf,
                         &h->nh_labels, &h->nh_keys, &h->nh_cnt, &h->nh_colcnt, &h->nh_diag, &h->nh_tmp, &h->nh_kf};
@@ -1673,7 +1673,9 @@ int gk_spattr_features(gk_handle* h, int32_t flags, gk_stats* stats) {
     LAUNCH_CHECK(h);
   }
   GK_TRY(h->diag_f64.ensure(N * 8));
-  rownorm_f64_kernel<<<(int)N, 256, 0, h->stream>>>(h->fattr.as<double>(), Dfeat, (int)N, h->diag_f64.as<double>());
+  GK_TRY(h->fattr_exp.ensure(N * 4));
+  rownorm_f64_kernel<<<(int)N, 256, 0, h->stream>>>(h->fattr.as<double>(), Dfeat, (int)N, h->diag_f64.as<double>(),
+                                                    h->fattr_exp.as<int>());
   LAUNCH_CHECK(h);
   GK_CUDA(cudaEventRecord(h->tev[3], h->stream));
   GK_CUDA(cudaStreamSynchronize(h->stream));  // host vectors above are sources of async copies
@@ -1698,9 +1700,11 @@ static void build_tiles(std::vector<int2>& tiles, int a0, int a1, int b0, int b1
 
 // Gram of the dense fp64 SP-attr feature matrix (feature_kind == 3).  Default: the tcgen05 kernel with tf32
 // operands on a hi/lo split of the features (3xTF32: hi hi^T + hi lo^T + lo hi^T, fp32 accumulation in TMEM,
-// k range processed in chunks and summed in fp64), self similarities exact in fp64; measured against the fp64
-// CUDA-core Gram (GRAKEL_B200_SPATTR_F64=1 selects it) the relative difference is ~1e-7, the north_star's
-// tolerance for real-valued Gram entries is 1e-5.
+// k range processed in chunks and summed in fp64), self similarities exact in fp64.  Every row is scaled by a power
+// of two before the split and K unscaled after it (spattr_split_tf32, unscale_gram_f64), so the range is fp64's and
+// K(2^s a) = 2^(4s) K(a) bit for bit.  Error bound: |K - K_exact| <= 1e-5 * <|phi_i|, |phi_j|> -- relative for
+// non-negative attributes (observed ~2e-6), normwise for signed ones, where cancelling entries can be far less
+// accurate relatively.  GRAKEL_B200_SPATTR_F64=1 selects the fp64 CUDA-core Gram for elementwise accuracy.
 static int gram_spattr(gk_handle* h, int64_t n_fit, int32_t flags, int64_t row_begin, int64_t row_end, void* K_out,
                        int32_t out_dtype, int64_t ld, double* xdiag, double* ydiag, gk_stats* stats) {
   if (out_dtype != GK_F64) return fail(GK_ERR_UNSUPPORTED, "ShortestPathAttr Gram is fp64 only");
@@ -1724,7 +1728,8 @@ static int gram_spattr(gk_handle* h, int64_t n_fit, int32_t flags, int64_t row_b
     GK_TRY(h->panel.ensure((size_t)N * W * 4 * 2));
     float* P1 = h->panel.as<float>();
     float* P2 = P1 + (size_t)N * W;
-    spattr_split_tf32<<<h->sm_count * 8, 256, 0, h->stream>>>(h->fattr.as<double>(), D, Dp, (int)N, P1, P2);
+    spattr_split_tf32<<<h->sm_count * 8, 256, 0, h->stream>>>(h->fattr.as<double>(), h->fattr_exp.as<int>(), D, Dp,
+                                                              (int)N, P1, P2);
     LAUNCH_CHECK(h);
     const bool sym = square && row_begin == 0 && row_end == N;
     std::vector<int2> tiles;
@@ -1744,7 +1749,7 @@ static int gram_spattr(gk_handle* h, int64_t n_fit, int32_t flags, int64_t row_b
     p.a_row_end = a1; p.b_row_end = (int)n_fit;
     p.c_row0 = a0; p.c_col0 = 0;
     p.out = h->K.p; p.ld = k_cols;
-    p.mirror = 0;  // the symmetric case mirrors the upper triangle once, after all chunks (mirror_upper_f64)
+    p.mirror = 0;  // the symmetric case mirrors the upper triangle once, after all chunks (unscale_gram_f64)
     p.diag = h->diag_f64.as<double>();
     // The tensor core's fp32 accumulate truncates (measured: -1.8e-5 relative for 960 sequential MMAs on all-positive
     // data, profiles/r02e_spattr_err.txt), so no accumulator sums more than `chunk` k-blocks x 4 MMAs: the kernel
@@ -1762,10 +1767,9 @@ static int gram_spattr(gk_handle* h, int64_t n_fit, int32_t flags, int64_t row_b
     const int grid = (int)std::min<size_t>(tiles.size(), h->sm_count);
     gram_tc_kernel<double, false, 1><<<grid, GEMM_THREADS, GEMM_SMEM, h->stream>>>(tmA, tmB, tmC, p);
     LAUNCH_CHECK(h);
-    if (sym) {
-      mirror_upper_f64<<<h->sm_count * 8, 256, 0, h->stream>>>((int)N, h->K.as<double>(), k_cols);
-      LAUNCH_CHECK(h);
-    }
+    unscale_gram_f64<<<h->sm_count * 8, 256, 0, h->stream>>>(a0, k_rows, k_cols, h->fattr_exp.as<int>(),
+                                                             h->K.as<double>(), k_cols, sym ? 1 : 0);
+    LAUNCH_CHECK(h);
     if (square) {  // exact self similarities
       set_diag_f64<<<cdiv(k_rows, 256), 256, 0, h->stream>>>(a0, a1, 0, (int)n_fit, h->diag_f64.as<double>(), h->K.as<double>(), k_cols);
       LAUNCH_CHECK(h);

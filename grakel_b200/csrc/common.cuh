@@ -195,6 +195,7 @@ struct gk_handle {
 
   // ---- SP-attr dense fp32 feature matrix
   gk::DevBuf fattr;
+  gk::DevBuf fattr_exp;  // [N] int: per-row scale exponent of the tensor-core split (rownorm_f64_kernel)
   int64_t fattr_dim = 0;
 
   // ---- GEMM

@@ -261,6 +261,9 @@ gram_f64_kernel(const double* __restrict__ phi, long long D, int a0, int a1, int
 // representable in tf32 (10 explicit mantissa bits: the low 13 bits of the fp32 pattern are zero after
 // round-to-nearest-even on bit 13).  K = hi hi^T + hi lo^T + lo hi^T is ONE GEMM over the concatenated
 // panels  P1 = [hi | hi | lo],  P2 = [hi | lo | hi]  (row pitch 3 * Dp floats, Dp = D rounded up to 32).
+// Row r is split as phi[r] * 2^-rexp[r] (exact in fp64; rexp from rownorm_f64_kernel), so its largest entry lies
+// in [1, 2) and hi, lo, their products and the fp32 chunk sums stay in fp32's normal range for any finite phi;
+// unscale_gram_f64 multiplies K[r][c] by 2^(rexp[r] + rexp[c]) afterwards.
 __device__ __forceinline__ float tf32_rne(float x) {
   unsigned u = __float_as_uint(x);
   u += 0x0FFFu + ((u >> 13) & 1u);
@@ -268,13 +271,14 @@ __device__ __forceinline__ float tf32_rne(float x) {
   return __uint_as_float(u);
 }
 __global__ void __launch_bounds__(256)
-spattr_split_tf32(const double* __restrict__ phi, long long D, long long Dp, int N, float* __restrict__ P1, float* __restrict__ P2) {
+spattr_split_tf32(const double* __restrict__ phi, const int* __restrict__ rexp, long long D, long long Dp, int N,
+                  float* __restrict__ P1, float* __restrict__ P2) {
   const long long total = (long long)N * Dp;
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
     const long long r = i / Dp, c = i - r * Dp;
     float hi = 0.f, lo = 0.f;
     if (c < D) {
-      const double x = phi[r * D + c];
+      const double x = ldexp(phi[r * D + c], -rexp[r]);
       hi = tf32_rne((float)x);
       lo = tf32_rne((float)(x - (double)hi));
     }
@@ -284,14 +288,20 @@ spattr_split_tf32(const double* __restrict__ phi, long long D, long long Dp, int
     p2[c] = hi; p2[Dp + c] = lo; p2[2 * Dp + c] = hi;
   }
 }
-// lower triangle := upper triangle (tiles that straddle the diagonal are written from both sides with values that may
-// differ in the last fp32 rounding of the accumulator; the reference's matrix is exactly symmetric, kernel.py:277)
+// K[r][c] *= 2^(rexp[a0 + r] + rexp[c]): undoes the row scaling of spattr_split_tf32 (exact unless the fp64 result
+// itself leaves fp64's range).  mirror (square, all rows, a0 = 0): the upper triangle is scaled and copied to the lower
+// one (tiles that straddle the diagonal are written from both sides with values that may differ in the last fp32
+// rounding of the accumulator; the reference's matrix is exactly symmetric, kernel.py:277).
 __global__ void __launch_bounds__(256)
-mirror_upper_f64(int n, double* __restrict__ out, long long ld) {
-  const long long total = (long long)n * n;
+unscale_gram_f64(int a0, long long rows, long long cols, const int* __restrict__ rexp, double* __restrict__ out,
+                 long long ld, int mirror) {
+  const long long total = rows * cols;
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
-    const int r = (int)(i / n), c = (int)(i - (long long)r * n);
-    if (r > c) out[(long long)r * ld + c] = out[(long long)c * ld + r];
+    const long long r = i / cols, c = i - r * cols;
+    if (mirror && r > c) continue;
+    const double v = ldexp(out[r * ld + c], rexp[a0 + r] + rexp[c]);
+    out[r * ld + c] = v;
+    if (mirror && r < c) out[c * ld + r] = v;
   }
 }
 // K[i][i] = diag[i] for the rows of a block (exact fp64 self similarities over the fp64 features)
@@ -301,22 +311,36 @@ set_diag_f64(int a0, int a1, int b0, int b1, const double* __restrict__ diag, do
   if (r < a1 && r >= b0 && r < b1) out[(long long)(r - a0) * ld + (r - b0)] = diag[r];
 }
 
-// per-row self similarity <phi[g], phi[g]>
+// per-row self similarity <phi[g], phi[g]>, and the row's scale exponent for spattr_split_tf32:
+// rexp[g] = ilogb(max_k |phi[g][k]|), 0 for an all-zero row or one with a non-finite entry (left as it is)
 __global__ void __launch_bounds__(256)
-rownorm_f64_kernel(const double* __restrict__ phi, long long D, int N, double* __restrict__ diag) {
+rownorm_f64_kernel(const double* __restrict__ phi, long long D, int N, double* __restrict__ diag, int* __restrict__ rexp) {
   const int g = blockIdx.x;
   if (g >= N) return;
-  __shared__ double red[8];
-  double s = 0.0;
-  for (long long k = threadIdx.x; k < D; k += 256) { const double x = phi[(long long)g * D + k]; s += x * x; }
+  __shared__ double red[8], redm[8];
+  __shared__ int redbad[8];
+  double s = 0.0, m = 0.0;
+  int bad = 0;
+  for (long long k = threadIdx.x; k < D; k += 256) {
+    const double x = phi[(long long)g * D + k];
+    s += x * x;
+    m = fmax(m, fabs(x));
+    bad |= !isfinite(x);
+  }
 #pragma unroll
-  for (int d = 16; d > 0; d >>= 1) s += __shfl_xor_sync(0xffffffffu, s, d);
-  if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = s;
+  for (int d = 16; d > 0; d >>= 1) {
+    s += __shfl_xor_sync(0xffffffffu, s, d);
+    m = fmax(m, __shfl_xor_sync(0xffffffffu, m, d));
+    bad |= __shfl_xor_sync(0xffffffffu, bad, d);
+  }
+  if ((threadIdx.x & 31) == 0) { red[threadIdx.x >> 5] = s; redm[threadIdx.x >> 5] = m; redbad[threadIdx.x >> 5] = bad; }
   __syncthreads();
   if (threadIdx.x == 0) {
-    double t = 0.0;
-    for (int w = 0; w < 8; ++w) t += red[w];
+    double t = 0.0, tm = 0.0;
+    int tb = 0;
+    for (int w = 0; w < 8; ++w) { t += red[w]; tm = fmax(tm, redm[w]); tb |= redbad[w]; }
     diag[g] = t;
+    rexp[g] = (tb || tm == 0.0) ? 0 : ilogb(tm);
   }
 }
 

@@ -469,9 +469,10 @@ def test_shortest_path_attr_matches_reference_loop(mode, monkeypatch):
     feature-map form on a config-5 shaped subset and SURVEY 8c's real-reference K[0,:5] of config 5.
 
     Default path: tcgen05 kind::tf32 GEMM on a hi/lo split of the fp64 features (3 passes, fp32 accumulation folded
-    into fp64 every few hundred MMAs); tolerance 1e-5 relative, the north_star's bound for real-valued Gram entries
-    (observed ~1e-7).  GRAKEL_B200_SPATTR_F64=1: the fp64 CUDA-core Gram, 1e-9.  Self similarities (the diagonal
-    and what normalisation divides by) are exact fp64 in both."""
+    into fp64 every few hundred MMAs, rows scaled by powers of two so the range is fp64's); error within 1e-5 of
+    sum_k |phi_ik| |phi_jk|, i.e. 1e-5 relative here, where the attributes are non-negative (observed ~2e-6; signed
+    attributes: normwise only, tests/test_spattr_edges.py).  GRAKEL_B200_SPATTR_F64=1: the fp64 CUDA-core Gram, 1e-9
+    elementwise.  Self similarities (the diagonal and what normalisation divides by) are exact fp64 in both."""
     from oracle.gk_oracle import SPAttrOracle
     tol = 1e-9 if mode == "fp64" else 1e-5
     if mode == "fp64":

@@ -109,6 +109,29 @@ def test_spattr():
     np.testing.assert_allclose(o.transform(Y), np.asarray(d["Ktn"]), rtol=1e-12)
 
 
+def test_spattr_dense_reference():
+    """tests/spattr_ref.py, the fp64 feature-matrix restatement the device ShortestPathAttr tests compare with
+    (K = Phi Phi^T), against the real reference: fit_transform / transform, raw and normalised, and the path sums in
+    Dijkstra's order on real-valued weights (its Floyd-Warshall twin gives a different matrix there)."""
+    import sys
+    from spattr_ref import spattr_ref
+    sys.path.insert(0, G)
+    from make_golden_dijkstra import gen_real
+    d = _load("spattr.json.gz")
+    X, Y = gio.dec_dataset(d["X"]), gio.dec_dataset(d["Y"])
+    for key, Yk, norm in (("K", None, False), ("Kt", Y, False), ("Kn", None, True), ("Ktn", Y, True)):
+        K, K_abs, drow, dcol = spattr_ref(X, Yk, normalize=norm)
+        np.testing.assert_allclose(K, np.asarray(d[key]), rtol=1e-12)
+        assert np.all(np.abs(K) <= K_abs * (1 + 1e-12))
+    K, K_abs, drow, dcol = spattr_ref(X)
+    assert np.array_equal(K, K.T) and np.array_equal(np.diagonal(K), drow) and np.array_equal(drow, dcol)
+    np.testing.assert_allclose(K_abs, K, rtol=1e-12)  # non-negative attributes: the error scale is K itself
+    A = gen_real(7, 8, 5, attr=3)
+    ref = np.load(os.path.join(G, "dijkstra_real.npz"))["attr_dj_K"]
+    np.testing.assert_allclose(spattr_ref(A, algorithm_type="dijkstra")[0], ref, rtol=1e-12)
+    assert not np.allclose(spattr_ref(A, algorithm_type="floyd_warshall")[0], ref, rtol=1e-6)
+
+
 def test_apsp_known_answer():
     """The reference's own APSP known-answer (grakel/tests/test_graph.py:40,62-65
     adjacency input with a self loop; :80-83,119-122 the same graph as a nested
